@@ -65,7 +65,27 @@ def parse():
                          "200x200x130; 5 = oriented IoU + NMS sweep 1k..1M boxes")
     ap.add_argument("--weights", default="spread", choices=["spread", "seed0"], help="headline weights: spread objectness (default) or plain seed-0 init")
     ap.add_argument("--rotated", action="store_true", help="headline with --rotated_bbox (8 deltas, OBB decode, polygon-clip NMS)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps of the default run (config 2 inference), write the last step's proposals, scores and levels of every "
+                         "scene as DIR/<name>.npy (float32), so that two builds can be compared output for output on the same seeded inputs; the other "
+                         "configurations and modes are comparison legs of their own and are not dumped")
+    args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.mode != "infer" or args.config != 2):
+        ap.error("--dump-outputs applies to the headline run (--impl b200 --mode infer --config 2)")
+    return args
+
+
+def dump_outputs(path, plan, prefix=""):
+    """What a caller of the engine receives from the last timed step: per scene, the proposals (count x 6 or 7), their objectness scores and
+    pyramid levels, as float32 .npy files (4 scenes x 2 500 proposals: well under 1 MB)."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    count = plan.out_count.cpu()
+    boxes, scores, levels = plan.out_boxes.cpu(), plan.out_scores.cpu(), plan.out_levels.cpu()
+    for b in range(count.numel()):
+        k = int(count[b])
+        for name, t in (("boxes", boxes), ("scores", scores), ("levels", levels)):
+            np.save(os.path.join(path, f"{prefix}scene{b}_{name}.npy"), t[b, :k].float().numpy())
 
 
 def synth_scene(i, layout="ncdhw"):
@@ -416,6 +436,8 @@ def run_b200(args):
     sampler = ClockSampler(local)
     ms, plan, count = device_throughput(model, dev, K, W, barrier, sampler if rank == 0 else None)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:                                  # before the pipeline below reuses the plan's output buffers
+        dump_outputs(args.dump_outputs, plan, f"rank{rank}_" if world > 1 else "")
 
     # ---- end to end through the streaming pipeline (pinned host grids in, proposals out on the host)
     with torch.no_grad():
@@ -701,7 +723,7 @@ def run_config(args):
             sets = [make(n, 10 * rank + k) for k in range(2)]                     # 2 x 32 MB at 1 M; the sort / grid scratch is ~0.5 GB: not L2-resident
             dev = [(b.cuda(), s.cuda()) for b, s in sets]
             pin = [(b.pin_memory(), s.pin_memory()) for b, s in sets]
-            reps = max(3, min(K, 2000000 // n))
+            reps = K                                                              # --steps timed repetitions at every size
             for i in range(W):
                 keep, nk = ops.nms_device(dev[i % 2][0], dev[i % 2][1], None, 0.3)
             barrier()

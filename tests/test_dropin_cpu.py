@@ -1,6 +1,6 @@
 """CPU: the drop-in shims make the reference's UNMODIFIED driver resolve `model.*` to this package and construct its model
-through our module mirror with the reference's own constructor calls (run_rpn.py:171-216, 274-292). Skipped on boxes without
-/root/reference (the GPU box)."""
+through our module mirror with the reference's own constructor calls (run_rpn.py:171-216, 274-292). They run the reference's own driver
+scripts, so they are skipped where the reference is not staged under oracle/_ref (oracle/build_ref.py)."""
 import os
 import subprocess
 import sys
@@ -8,11 +8,13 @@ import textwrap
 
 import pytest
 
+from oracle.build_ref import ref_root
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference/nerf_rpn"
+REF = ref_root() or ""
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout not present")
+@pytest.mark.skipif(not os.path.isdir(REF), reason="oracle/_ref not staged")
 @pytest.mark.parametrize("backbone", ["resnet", "vgg_EF", "swin_s"])
 def test_reference_driver_builds_our_modules(backbone, tmp_path):
     code = textwrap.dedent(f"""
@@ -42,7 +44,7 @@ def test_reference_driver_builds_our_modules(backbone, tmp_path):
     assert "OK" in r.stdout
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout not present")
+@pytest.mark.skipif(not os.path.isdir(REF), reason="oracle/_ref not staged")
 def test_reference_fcos_driver_builds_our_modules(tmp_path):
     code = textwrap.dedent(f"""
         import sys, types

@@ -1,6 +1,7 @@
 """GPU: the training-step kernels (csrc/train.cu, generalised wgrad) against plain PyTorch fp32 autograd of the same op, and the whole
 training step (nerf_rpn_b200/train.py) against the UNMODIFIED reference's own `model(rgbsigma, boxes)` + `loss.backward()` run in fp32
-on the same GPU (oracle/_ref).  Tolerances are stated per test: 16-bit activations / gradients, fp32 accumulation."""
+on a B200: the loss tests against its results stored under tests/golden/reference/ (tests/reference_golden.py); the whole-step parity tests
+against the reference itself, staged under oracle/_ref (their whole-gradient metrics need every gradient value of the reference).  Tolerances are stated per test: 16-bit activations / gradients, fp32 accumulation."""
 import ctypes
 import math
 import os
@@ -10,7 +11,11 @@ import pytest
 import torch
 import torch.nn.functional as F
 
+from tests.reference_golden import recorded, recording
+
 pytestmark = pytest.mark.gpu
+ANCHOR_SIZES = ((8,), (16,), (32,), (64,),)
+ASPECT = (((1., 1., 1.), (1., 1., 2.), (1., 2., 2.), (1., 1., 3.), (1., 3., 3.)),) * 4
 
 
 def _p(t):
@@ -290,6 +295,35 @@ def _grad_metrics(grads, ref):
     return F.cosine_similarity(fg, fr, dim=0).item(), ((fg - fr).norm() / fr.norm()).item(), per
 
 
+def _our_model(layers, rotated, **kw):
+    """Our module mirror with the reference's seed-0 init (run_rpn.py's order: backbone, anchor generator, head)."""
+    from nerf_rpn_b200.model.anchor import AnchorGenerator3D, RPNHead
+    from nerf_rpn_b200.model.feature_extractor import Bottleneck, ResNet_FPN_256
+    from nerf_rpn_b200.model.nerf_rpn import NeRFRegionProposalNetwork
+    torch.manual_seed(0)
+    backbone = ResNet_FPN_256(Bottleneck, list(layers), input_dim=4, is_max_pool=True)
+    ag = AnchorGenerator3D(ANCHOR_SIZES, ASPECT)
+    head = RPNHead(256, 13, 4, rotate=rotated)
+    return backbone, head, NeRFRegionProposalNetwork(backbone, ag, head, rpn_fg_iou_thresh=0.35, rpn_bg_iou_thresh=0.2, rotated_bbox=rotated, **kw)
+
+
+def _linearised(w, pos, deltas):
+    """The reference's loss and gradient at the engine's deltas, from its values at the deltas stored with them: first order around those
+    (the sampled positives must be the same and the deltas within 1 % of their scale -- 16-bit forward noise -- for that to hold)."""
+    assert torch.equal(pos.cpu(), torch.from_numpy(w["pos"]).to(pos.dtype)), "the sampled positives differ from the stored ones"
+    d0, g0 = torch.from_numpy(w["deltas"]).cuda(), torch.from_numpy(w["gwant"]).cuda()
+    dd = deltas - d0
+    assert dd.abs().max().item() <= 1e-2 * d0.abs().max().item(), dd.abs().max().item()
+    return torch.tensor(float(w["want"]), dtype=torch.float64) + (g0.double() * dd.double()).sum().cpu(), g0
+
+
+def _same_weights(backbone, head, rm):
+    """Recording only: our seeded init equals the reference's."""
+    for ours, theirs in ((backbone, rm.backbone), (head, rm.rpn.head)):         # parameters: the reference has already run a training forward
+        ref_params = dict(theirs.named_parameters())
+        assert all(torch.equal(v.detach().cpu(), ref_params[k].detach().cpu()) for k, v in ours.named_parameters())
+
+
 @pytest.mark.parametrize("layers,rotated,precision", [((2, 1, 1, 1), True, "fp16"), ((2, 1, 1, 1), False, "bf16"), ((3, 4, 6, 3), True, "bf16"), ((3, 4, 6, 3), False, "fp16")])
 def test_training_step_vs_reference_autograd(layers, rotated, precision):
     _training_step_parity(layers, rotated, precision, (64, 96, 80), 12)
@@ -378,28 +412,23 @@ def test_iou_regression_loss_vs_reference_rotated_iou_loss(loss_type):
     deltas against the REFERENCE's own coder + RotatedIOULoss + autograd evaluated on the engine's fp32 deltas, same sampled positives; and the whole
     step's regression loss against the reference network in fp32 (feature noise of the 16-bit forward only)."""
     from oracle import ref_gpu
-    if not ref_gpu.available():
-        pytest.skip("oracle/_ref not staged")
-    from nerf_rpn_b200.model.anchor import AnchorGenerator3D, RPNHead
-    from nerf_rpn_b200.model.feature_extractor import Bottleneck, ResNet_FPN_256
-    from nerf_rpn_b200.model.nerf_rpn import NeRFRegionProposalNetwork
     from nerf_rpn_b200.train import RPNTrainEngine
     layers, dims = (2, 1, 1, 1), (64, 96, 80)
     grid, gt = _planted(dims, 12, 11, True)
     grid, gt = grid.cuda(), gt.cuda()
-    rm = ref_gpu.build_reference_model(rotated=True, seed=0, layers=layers, rpn_fg_iou_thresh=0.35, rpn_bg_iou_thresh=0.2, reg_loss_type=loss_type).cuda().train()
-    old = (torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32)
-    torch.backends.cudnn.allow_tf32 = False; torch.backends.cuda.matmul.allow_tf32 = False
-    try:
-        torch.manual_seed(123)
-        _, ref_losses, _ = rm([grid], [gt])
-    finally:
-        torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32 = old
-    backbone = ResNet_FPN_256(Bottleneck, list(layers), input_dim=4, is_max_pool=True)
-    head = RPNHead(256, 13, 4, rotate=True)
-    backbone.load_state_dict(rm.backbone.state_dict()); head.load_state_dict(rm.rpn.head.state_dict())
-    model = NeRFRegionProposalNetwork(backbone, AnchorGenerator3D(ref_gpu.ANCHOR_SIZES, ref_gpu.ASPECT), head, rpn_fg_iou_thresh=0.35, rpn_bg_iou_thresh=0.2,
-                                      rotated_bbox=True, reg_loss_type=loss_type).cuda().train()
+    if recording():
+        rm = ref_gpu.build_reference_model(rotated=True, seed=0, layers=layers, rpn_fg_iou_thresh=0.35, rpn_bg_iou_thresh=0.2, reg_loss_type=loss_type).cuda().train()
+        old = (torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32)
+        torch.backends.cudnn.allow_tf32 = False; torch.backends.cuda.matmul.allow_tf32 = False
+        try:
+            torch.manual_seed(123)
+            _, ref_losses, _ = rm([grid], [gt])
+        finally:
+            torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32 = old
+    backbone, head, model = _our_model(layers, True, reg_loss_type=loss_type)
+    if recording():
+        _same_weights(backbone, head, rm)
+    model = model.cuda().train()
     eng = RPNTrainEngine(model, precision="fp16", lr=1e-4, weight_decay=0.01, clip_grad_norm=0.1, reg_loss_weight=5.0)
     plan = eng.plan(1, dims)
     torch.manual_seed(123)
@@ -408,7 +437,7 @@ def test_iou_regression_loss_vs_reference_rotated_iou_loss(loss_type):
     pos, neg, gtp = plan.last_samples[0]
     assert pos.numel() >= 8
     norm = float(pos.numel() + neg.numel())
-    # the engine's own deltas of the sampled positives (fp32 predictor output), decoded and scored by the REFERENCE's code
+    # the engine's own deltas of the sampled positives (fp32 predictor output)
     A, code = eng.A, 8
     level, vox, a = plan._split_anchor_index(pos)
     cols = (A + a * code).view(-1, 1) + torch.arange(code, device=pos.device).view(1, -1)
@@ -419,15 +448,21 @@ def test_iou_regression_loss_vs_reference_rotated_iou_loss(loss_type):
         if m.any():
             deltas[m] = plan.pred_levels[l][0].reshape(-1, 128)[vox[m].view(-1, 1), cols[m]]
             dgot[m] = plan.dpred_levels[l][0].reshape(-1, 128)[vox[m].view(-1, 1), cols[m]].float()
-    d = deltas.clone().requires_grad_(True)
-    boxes = rm.rpn.box_coder.decode_single(d, plan._anchors()[pos])
-    want = rm.rpn.rotated_iou_loss(boxes, gtp) / norm
-    (gwant,) = torch.autograd.grad(want, d)
+
+    def reference():                                         # the REFERENCE's coder + RotatedIOULoss + autograd on these deltas
+        d = deltas.clone().requires_grad_(True)
+        boxes = rm.rpn.box_coder.decode_single(d, plan._anchors()[pos])
+        want = rm.rpn.rotated_iou_loss(boxes, gtp) / norm
+        (gwant,) = torch.autograd.grad(want, d)
+        return dict(net_loss=ref_losses["loss_rpn_box_reg"].item(), pos=pos.cpu().numpy(), deltas=deltas.cpu().numpy(), want=want.item(), gwant=gwant.cpu().numpy())
+    w = recorded(f"iou_regression_loss_{loss_type}", reference)
+    want, gwant = _linearised(w, pos, deltas)
+    ref_net = float(w["net_loss"])
     got_loss = float(out[1])
     print(f"[{loss_type}] regression loss: engine {got_loss:.6f}  reference code on the engine's deltas {want.item():.6f}  reference network fp32 "
-          f"{ref_losses['loss_rpn_box_reg'].item():.6f}  ({pos.numel()} positives)")
+          f"{ref_net:.6f}  ({pos.numel()} positives)")
     assert abs(got_loss - want.item()) <= 2e-4 * abs(want.item()) + 1e-7
-    assert abs(got_loss - ref_losses["loss_rpn_box_reg"].item()) <= 0.05 * abs(ref_losses["loss_rpn_box_reg"].item())
+    assert abs(got_loss - ref_net) <= 0.05 * abs(ref_net)
     scale = 5.0 * eng.loss_scale
     err = (dgot / scale - gwant).abs().max().item()
     print(f"[{loss_type}] d loss / d deltas: max abs err {err:.3e} of scale {gwant.abs().max().item():.3e}")
@@ -442,27 +477,22 @@ def test_projection_2d_loss_vs_reference(rotated):
     coder + get_w2cs / project / obb2points_3d + autograd evaluated on the engine's fp32 deltas (same sampled positives); the whole step's value against
     the reference network in fp32; and the drop-in loop (losses dict with a grad_fn, weight applied outside the model as run_rpn.py:385-387 does)."""
     from oracle import ref_gpu
-    if not ref_gpu.available():
-        pytest.skip("oracle/_ref not staged")
-    from nerf_rpn_b200.model.anchor import AnchorGenerator3D, RPNHead
-    from nerf_rpn_b200.model.feature_extractor import Bottleneck, ResNet_FPN_256
-    from nerf_rpn_b200.model.nerf_rpn import NeRFRegionProposalNetwork
     from nerf_rpn_b200.train import RPNTrainEngine
-    ref = ref_gpu.load()
     layers, dims = (2, 1, 1, 1), (64, 96, 80)
     grid, gt = _planted(dims, 12, 11, rotated)
     grid, gt = grid.cuda(), gt.cuda()
-    rm = ref_gpu.build_reference_model(rotated=rotated, seed=0, layers=layers, rpn_fg_iou_thresh=0.35, rpn_bg_iou_thresh=0.2).cuda().train()
     old = (torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32)
     torch.backends.cudnn.allow_tf32 = False; torch.backends.cuda.matmul.allow_tf32 = False
     try:
-        torch.manual_seed(123)
-        _, ref_losses, _ = rm([grid], [gt])
-        backbone = ResNet_FPN_256(Bottleneck, list(layers), input_dim=4, is_max_pool=True)
-        head = RPNHead(256, 13, 4, rotate=rotated)
-        backbone.load_state_dict(rm.backbone.state_dict()); head.load_state_dict(rm.rpn.head.state_dict())
-        model = NeRFRegionProposalNetwork(backbone, AnchorGenerator3D(ref_gpu.ANCHOR_SIZES, ref_gpu.ASPECT), head, rpn_fg_iou_thresh=0.35, rpn_bg_iou_thresh=0.2,
-                                          rotated_bbox=rotated).cuda().train()
+        if recording():
+            ref = ref_gpu.load()
+            rm = ref_gpu.build_reference_model(rotated=rotated, seed=0, layers=layers, rpn_fg_iou_thresh=0.35, rpn_bg_iou_thresh=0.2).cuda().train()
+            torch.manual_seed(123)
+            _, ref_losses, _ = rm([grid], [gt])
+        backbone, head, model = _our_model(layers, rotated)
+        if recording():
+            _same_weights(backbone, head, rm)
+        model = model.cuda().train()
         w2d = 0.7
         eng = RPNTrainEngine(model, precision="fp16", lr=1e-4, weight_decay=0.01, clip_grad_norm=0.1, reg_loss_weight=0.0, reg_loss_weight_2d=w2d)
         plan = eng.plan(1, dims)
@@ -477,27 +507,32 @@ def test_projection_2d_loss_vs_reference(rotated):
             m = level == l
             if m.any():
                 dgot[m] = plan.dpred_levels[l][0].reshape(-1, 128)[vox[m].view(-1, 1), cols[m]].float()
-        # the reference's own pieces on the engine's deltas
-        d = deltas.clone().requires_grad_(True)
-        boxes = rm.rpn.box_coder.decode_single(d, plan._anchors()[pos])
-        res = max(dims)
-        if rotated:
-            from_ref = ref.rpn.obb2points_3d
-            p3, t3 = from_ref(boxes), from_ref(gtp)
-        else:
-            p3, t3 = torch.cat([boxes[:, :3], boxes[:, 3:]], 0), torch.cat([gtp[:, :3], gtp[:, 3:]], 0)
-        ones = torch.ones(p3.shape[0], 1, device="cuda")
-        K = torch.tensor([[600.0, 0, 320.0], [0, 600.0, 240.0], [0, 0, 1.0]], device="cuda")
-        pp, tt = [], []
-        for pose in ref.rpn.get_w2cs(res=res):
-            pp.append(ref.rpn.project(K, pose, torch.cat([p3, ones], 1))); tt.append(ref.rpn.project(K, pose, torch.cat([t3, ones], 1)))
-        want = F.smooth_l1_loss(torch.cat(pp), torch.cat(tt), beta=1 / 9, reduction="sum") / pos.numel() / res
-        (gwant,) = torch.autograd.grad(want, d)
+
+        def reference():                                     # the reference's own pieces on these deltas
+            d = deltas.clone().requires_grad_(True)
+            boxes = rm.rpn.box_coder.decode_single(d, plan._anchors()[pos])
+            res = max(dims)
+            if rotated:
+                p3, t3 = ref.rpn.obb2points_3d(boxes), ref.rpn.obb2points_3d(gtp)
+            else:
+                p3, t3 = torch.cat([boxes[:, :3], boxes[:, 3:]], 0), torch.cat([gtp[:, :3], gtp[:, 3:]], 0)
+            ones = torch.ones(p3.shape[0], 1, device="cuda")
+            K = torch.tensor([[600.0, 0, 320.0], [0, 600.0, 240.0], [0, 0, 1.0]], device="cuda")
+            pp, tt = [], []
+            for pose in ref.rpn.get_w2cs(res=res):
+                pp.append(ref.rpn.project(K, pose, torch.cat([p3, ones], 1))); tt.append(ref.rpn.project(K, pose, torch.cat([t3, ones], 1)))
+            want = F.smooth_l1_loss(torch.cat(pp), torch.cat(tt), beta=1 / 9, reduction="sum") / pos.numel() / res
+            (gwant,) = torch.autograd.grad(want, d)
+            return dict(net_loss=ref_losses["loss_rpn_box_reg_2d"].item(), pos=pos.cpu().numpy(), deltas=deltas.cpu().numpy(), want=want.item(),
+                        gwant=gwant.cpu().numpy())
+        w = recorded(f"projection_2d_loss_{'obb' if rotated else 'aabb'}", reference)
+        want, gwant = _linearised(w, pos, deltas)
+        ref_net = float(w["net_loss"])
         got = eng.loss_2d.item()
         print(f"[2d rotated={rotated}] engine {got:.6f}  reference code on the engine's deltas {want.item():.6f}  reference network fp32 "
-              f"{ref_losses['loss_rpn_box_reg_2d'].item():.6f}  ({pos.numel()} positives)")
+              f"{ref_net:.6f}  ({pos.numel()} positives)")
         assert abs(got - want.item()) <= 1e-4 * abs(want.item()) + 1e-7
-        assert abs(got - ref_losses["loss_rpn_box_reg_2d"].item()) <= 0.05 * abs(ref_losses["loss_rpn_box_reg_2d"].item())
+        assert abs(got - ref_net) <= 0.05 * abs(ref_net)
         err = (dgot / (w2d * eng.loss_scale) - gwant).abs().max().item()
         print(f"[2d rotated={rotated}] d loss / d deltas: max abs err {err:.3e} of scale {gwant.abs().max().item():.3e}")
         assert err <= 1e-2 * gwant.abs().max().item()                      # d(pred) is 16-bit
@@ -511,7 +546,7 @@ def test_projection_2d_loss_vs_reference(rotated):
         torch.manual_seed(123)
         _, losses, _ = model([grid], [gt])
         l2d = losses["loss_rpn_box_reg_2d"]
-        assert l2d.requires_grad and abs(l2d.item() - ref_losses["loss_rpn_box_reg_2d"].item()) <= 0.1 * abs(ref_losses["loss_rpn_box_reg_2d"].item())
+        assert l2d.requires_grad and abs(l2d.item() - ref_net) <= 0.1 * abs(ref_net)
         losses["loss_rpn_box_reg"] *= 5.0
         losses["loss_rpn_box_reg_2d"] *= 0.3
         (losses["loss_objectness"] + losses["loss_rpn_box_reg"] + losses["loss_rpn_box_reg_2d"]).backward()

@@ -35,6 +35,9 @@ def test_net_oracle_matches_reference(golden_dir, name, rot):
     for i in range(4):
         np.testing.assert_allclose(logits[i][0].numpy(), g[f"logits{i}"], rtol=1e-3, atol=2e-3)
     assert b.shape == g["proposals"].shape
+    if rot:                        # a yaw on the +-pi/2 boundary can come out at either end after last-bit differences: the same box
+        b = np.array(b, dtype=np.float64)
+        b[:, 6] -= np.pi * np.round((b[:, 6] - g["proposals"][:, 6]) / np.pi)
     np.testing.assert_allclose(b, g["proposals"], rtol=1e-3, atol=1e-2)
     np.testing.assert_array_equal(lv, g["level_index"])
 
