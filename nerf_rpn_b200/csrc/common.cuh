@@ -60,6 +60,12 @@ __device__ __forceinline__ float2 unpack_act2(uint32_t u, int fp16) {
     if (fp16) return __half22float2(*reinterpret_cast<const __half2*>(&u));
     return __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&u));
 }
+// max that propagates NaN, as torch's max-pooling does (fmaxf drops it): one max.NaN instruction
+__device__ __forceinline__ float max_nan(float a, float b) {
+    float r;
+    asm("max.NaN.f32 %0, %1, %2;" : "=f"(r) : "f"(a), "f"(b));
+    return r;
+}
 #endif
 
 template <typename T>

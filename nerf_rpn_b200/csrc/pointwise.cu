@@ -102,7 +102,8 @@ __global__ void pack_stem_cl_u8_kernel(const uint32_t* __restrict__ grid, int n,
     }
 }
 
-// F.max_pool3d(k=3, s=2, p=1) on channels-last bf16; one thread per (output voxel, 8 channels).
+// F.max_pool3d(k=3, s=2, p=1) on channels-last bf16; one thread per (output voxel, 8 channels).  A NaN in the window makes
+// the output NaN, as in torch.
 __global__ void maxpool_k3s2_kernel(const __nv_bfloat16* __restrict__ in, int n, int X, int Y, int Z, int C, int Xo, int Yo,
                                     int Zo, __nv_bfloat16* __restrict__ out, int fp16) {
     const int cg = C >> 3;
@@ -134,7 +135,7 @@ __global__ void maxpool_k3s2_kernel(const __nv_bfloat16* __restrict__ in, int n,
                 for (int dz = 0; dz < 3; ++dz) {
                     const uint32_t* h = reinterpret_cast<const uint32_t*>(&raw[dz]);
 #pragma unroll
-                    for (int q = 0; q < 4; ++q) { const float2 f = unpack_act2(h[q], fp16); m[2 * q] = fmaxf(m[2 * q], f.x); m[2 * q + 1] = fmaxf(m[2 * q + 1], f.y); }
+                    for (int q = 0; q < 4; ++q) { const float2 f = unpack_act2(h[q], fp16); m[2 * q] = max_nan(m[2 * q], f.x); m[2 * q + 1] = max_nan(m[2 * q + 1], f.y); }
                 }
             }
         }
@@ -146,7 +147,7 @@ __global__ void maxpool_k3s2_kernel(const __nv_bfloat16* __restrict__ in, int n,
 }
 
 // nn.MaxPool3d(kernel 2, stride 2, ceil_mode=True) on channels-last bf16 (VGG stages, feature_extractor.py:347):
-// output extent ceil(in/2); the last window is clipped at the border.
+// output extent ceil(in/2); the last window is clipped at the border.  NaN propagates, as in torch.
 __global__ void maxpool_k2s2_ceil_kernel(const __nv_bfloat16* __restrict__ in, int n, int X, int Y, int Z, int C, int Xo, int Yo,
                                          int Zo, __nv_bfloat16* __restrict__ out, int fp16) {
     const int cg = C >> 3;
@@ -171,7 +172,7 @@ __global__ void maxpool_k2s2_ceil_kernel(const __nv_bfloat16* __restrict__ in, i
                     const uint4 raw = __ldg(reinterpret_cast<const uint4*>(in + ((((size_t)b * X + x) * Y + y) * Z + z) * C + g * 8));
                     const uint32_t* h = reinterpret_cast<const uint32_t*>(&raw);
 #pragma unroll
-                    for (int q = 0; q < 4; ++q) { const float2 f = unpack_act2(h[q], fp16); m[2 * q] = fmaxf(m[2 * q], f.x); m[2 * q + 1] = fmaxf(m[2 * q + 1], f.y); }
+                    for (int q = 0; q < 4; ++q) { const float2 f = unpack_act2(h[q], fp16); m[2 * q] = max_nan(m[2 * q], f.x); m[2 * q + 1] = max_nan(m[2 * q + 1], f.y); }
                 }
             }
         }

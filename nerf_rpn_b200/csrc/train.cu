@@ -215,7 +215,8 @@ __global__ void __launch_bounds__(256) bn_backward_apply_kernel(const __nv_bfloa
 
 // ---------------------------------------------------------------------------------------------- max-pool (3,2,1) with argmax
 // Forward: out = max over the 3^3 window; idx = window position (dx+1)*9 + (dy+1)*3 + (dz+1) of the FIRST maximum in scan order
-// (x outer, z inner; padded taps skipped) -- the element torch's max_pool3d_with_indices records.
+// (x outer, z inner; padded taps skipped), or of the LAST NaN, which then is the output -- the element torch's
+// max_pool3d_with_indices records (its test is `val > max || isnan(val)`).
 __global__ void __launch_bounds__(256) maxpool_k3s2_argmax_kernel(const __nv_bfloat16* __restrict__ in, int n, int X, int Y, int Z, int C, int Xo, int Yo,
                                                                   int Zo, __nv_bfloat16* __restrict__ out, uint8_t* __restrict__ idx, int fp16) {
     const int cg = C >> 3;
@@ -241,8 +242,8 @@ __global__ void __launch_bounds__(256) maxpool_k3s2_argmax_kernel(const __nv_bfl
 #pragma unroll
                     for (int q = 0; q < 4; ++q) {
                         const float2 f = unpack_act2(h[q], fp16);
-                        if (f.x > m[2 * q]) { m[2 * q] = f.x; am[2 * q] = code; }
-                        if (f.y > m[2 * q + 1]) { m[2 * q + 1] = f.y; am[2 * q + 1] = code; }
+                        if (f.x > m[2 * q] || isnan(f.x)) { m[2 * q] = f.x; am[2 * q] = code; }
+                        if (f.y > m[2 * q + 1] || isnan(f.y)) { m[2 * q + 1] = f.y; am[2 * q + 1] = code; }
                     }
                 }
             }

@@ -331,7 +331,7 @@ def pack_stem_input(grid: torch.Tensor, out: Optional[torch.Tensor] = None, dtyp
     `grid` may be contiguous NCDHW or the channels-last view the reference's dataset yields (memory (N,X,Y,Z,4))."""
     if isinstance(grid, torch.Tensor) and grid.is_cuda and grid.dtype == torch.uint8 and grid.dim() == 5:
         # raw uint8 grid in its on-disk order: normalised (/ 255) on the device
-        if not is_channels_last_grid(grid):
+        if not grid.permute(0, 2, 3, 4, 1).is_contiguous():
             raise ValueError("nerf_rpn_b200: uint8 grids must be the (N,4,X,Y,Z) view of a contiguous (N,X,Y,Z,4) array")
         n, c, x, y, z = grid.shape
         shape = (n, (x + 1) // 2, (y + 1) // 2, (z + 1) // 2 + 1, 64)
